@@ -2,7 +2,7 @@
 """bench.py -- rays/sec of the layered ray-march hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--precision exact|exact_cf|mixed|fp32|fast]
-                    [--workload taekwondo2|walking4|walking6_4k] [--no-extra] [--no-cpu-baseline]
+                    [--workload taekwondo2|walking4|walking6_4k] [--no-extra] [--no-cpu-baseline] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): taekwondo 2-layer scene, 1080p, 16 views, 64 coarse + 128 fine samples.
 A *step* renders one 1080p view (2 073 600 rays; view = step mod 16) through the whole hot path: ray generation ->
@@ -231,8 +231,35 @@ def cpu_leg_parity(wl, model, dev, precision="exact"):
                        "instability of the reference) in tests/test_gpu_parity_scale.py" % wl["fixture"]}
 
 
-def measure(wl, precision, steps, warmup, rank, world, local_rank, want_e2e=True, parity_fn=None):
-    """One workload on this process' GPU (all ranks call it).  Returns a dict of measurements (complete on rank 0)."""
+DUMP_BYTES_PER_ARRAY = 30 * 10**6    # two arrays stay under 64 MB together
+
+
+def dump_outputs(out_dir, svr, rows, rank, world):
+    """Writes the fine and coarse images of the last timed step (every plane: merged + per layer; rgb, depth, acc) as
+    float32 `fine_images.npy` / `coarse_images.npy` of shape (planes, pixels, 5).  Where a full view is larger than the
+    budget, the same seeded sample of pixels (ascending flat indices) is taken from both."""
+    import numpy as np
+    import torch
+    from stnerf_b200.dist import all_gather_inplace, rows_view
+    coarse_local = svr._coarse[1]                               # (1, planes, rows_pad*W, 5): this rank's rows only
+    coarse = coarse_local.new_zeros((world,) + tuple(coarse_local.shape))
+    coarse[rank].copy_(coarse_local)
+    all_gather_inplace(coarse, rank, world)
+    if rank != 0:
+        return
+    images = {"fine_images": svr.assembled(rows)[0], "coarse_images": svr.assembled(rows_view(coarse, svr.W))[0]}
+    planes, hw = images["fine_images"].shape[0], svr.H * svr.W
+    n = min(hw, DUMP_BYTES_PER_ARRAY // (planes * 5 * 4))
+    idx = torch.arange(hw) if n == hw else torch.randperm(hw, generator=torch.Generator().manual_seed(0))[:n].sort()[0]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, img in images.items():
+        a = img.reshape(planes, hw, 5)[:, idx.to(img.device)].float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure(wl, precision, steps, warmup, rank, world, local_rank, want_e2e=True, parity_fn=None, dump_dir=None):
+    """One workload on this process' GPU (all ranks call it).  Returns a dict of measurements (complete on rank 0).
+    `dump_dir`: write the images of the last timed step there (dump_outputs)."""
     import torch
     import torch.distributed as dist
     import stnerf_b200 as S
@@ -267,24 +294,28 @@ def measure(wl, precision, steps, warmup, rank, world, local_rank, want_e2e=True
     if world > 1:
         dist.barrier()
     clocks = ClockSampler(local_rank); clocks.start()
-    launches0 = S.launch_count()
-    nat.profile_begin()
-    torch.cuda.synchronize()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    coll_ms = []
-    e0.record()
-    for i in range(steps):
-        step(warmup + i)
+    try:                                              # the sampler's nvidia-smi child must not outlive a failed run
+        launches0 = S.launch_count()
+        nat.profile_begin()
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        coll_ms = []
+        e0.record()
+        for i in range(steps):
+            rows = step(warmup + i)
+            if world > 1:
+                coll_ms.append(svr._timing)
+        e1.record()
+        torch.cuda.synchronize()
         if world > 1:
-            coll_ms.append(svr._timing)
-    e1.record()
-    torch.cuda.synchronize()
-    if world > 1:
-        dist.barrier()
-    ms_total = e0.elapsed_time(e1)
-    prof = nat.profile_end()
-    launches = S.launch_count() - launches0
-    clk = clocks.stop()
+            dist.barrier()
+        ms_total = e0.elapsed_time(e1)
+        prof = nat.profile_end()
+        launches = S.launch_count() - launches0
+    finally:
+        clk = clocks.stop()
+    if dump_dir is not None:
+        dump_outputs(dump_dir, svr, rows, rank, world)
     t = torch.tensor([ms_total], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -386,7 +417,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the short runs of the other BASELINE configs")
     ap.add_argument("--workload", default="taekwondo2", choices=list(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the fine and coarse images of the last timed step as DIR/<name>.npy (float32, a seeded pixel "
+                         "sample where a view exceeds 30 MB per array), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -419,7 +455,8 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     # the reference-fixture parity check belongs to the CPU leg: rank 0 of a single-GPU run, unless --no-cpu-baseline
     parity_fn = cpu_leg_parity if (world == 1 and not args.no_cpu_baseline) else None
-    res = measure(wl, args.precision, args.steps, args.warmup, rank, world, local_rank, parity_fn=parity_fn)
+    res = measure(wl, args.precision, args.steps, args.warmup, rank, world, local_rank, parity_fn=parity_fn,
+                  dump_dir=args.dump_outputs)
 
     extra = {}
     if not args.no_extra and args.workload == "taekwondo2":

@@ -233,6 +233,16 @@ def drive_camera_path(r, sc):
         r.invert_poses()
 
 
+CHECKPOINT_FILE_NAMES = ("layered_rfnr_checkpoint_3.pt", "layered_rfnr_checkpoint_12.pt", "layered_rfnr_checkpoint_5_200.pt",
+                         "other.pt")
+
+
+def camera_file_inputs():
+    """Rows of K.txt (5, 9) and camera poses (5, 12) for the camera-file parsers (checkpoint_io.npz)."""
+    rs = np.random.RandomState(3)
+    return rs.rand(5, 9) * 1000, rs.rand(5, 12)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # Synthetic captured-scene directory (SURVEY 8f row 4): the files FrameLayerDataset / Ray_Dataset_Render read.
 # ---------------------------------------------------------------------------------------------------------------------

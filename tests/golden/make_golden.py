@@ -214,13 +214,37 @@ def run_dataset():
     print("dataset.npz: %d arrays" % len(out))
 
 
+def run_checkpoint_io():
+    """data/datasets/utils.py (numpy only): checkpoint discovery and camera-file parsing on cases.CHECKPOINT_FILE_NAMES /
+    cases.camera_file_inputs().  Paths are stored relative to the checkpoint directory."""
+    import importlib.util, tempfile
+    spec = importlib.util.spec_from_file_location("_ref_dataset_utils", os.path.join(R.REFERENCE_ROOT, "data", "datasets", "utils.py"))
+    ref = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(ref)
+    d = tempfile.mkdtemp(prefix="stnerf_ckpt_")
+    for name in C.CHECKPOINT_FILE_NAMES:
+        open(os.path.join(d, name), "w").close()
+    Ks, poses = C.camera_file_inputs()
+    fn = os.path.join(d, "K.txt")
+    np.savetxt(fn, Ks)
+    assert ref.get_iteration_path(os.path.join(d, "nope")) is None
+    out = dict(iteration_path=np.array(os.path.relpath(ref.get_iteration_path(d), d)),
+               iteration_path_fix7=np.array(os.path.relpath(ref.get_iteration_path(d, 7), d)),
+               intrinsics=ref.read_intrinsics(fn), extrinsics=ref.campose_to_extrinsic(poses))
+    shutil.rmtree(d, ignore_errors=True)
+    np.savez_compressed(os.path.join(HERE, "checkpoint_io.npz"), **out)
+    print("checkpoint_io.npz: %d arrays" % len(out))
+
+
 if __name__ == "__main__":
     assert R.available(), "needs /root/reference (build container only)"
     torch.set_num_threads(os.cpu_count())
     stash_checkpoints()
-    names = sys.argv[1:] or (list(C.CASES) + ["functions", "camera_path", "dataset"])
+    names = sys.argv[1:] or (list(C.CASES) + ["functions", "camera_path", "dataset", "checkpoint_io"])
     for nm in names:
-        if nm == "functions":
+        if nm == "checkpoint_io":
+            run_checkpoint_io()
+        elif nm == "functions":
             run_functions()
         elif nm == "camera_path":
             run_camera_path()

@@ -1,6 +1,5 @@
-"""Checkpoint discovery / loading and camera-file parsing (SURVEY 8f rows 3-4).  CPU only.  When the reference tree is
-present (build container) its own functions (data/datasets/utils.py, a numpy-only module) are executed side by side."""
-import importlib.util
+"""Checkpoint discovery / loading and camera-file parsing (SURVEY 8f rows 3-4).  CPU only.  checkpoint_io.npz holds what
+the reference's own functions (data/datasets/utils.py) return for the same inputs (tests/golden/make_golden.py)."""
 import os
 
 import numpy as np
@@ -10,52 +9,35 @@ import torch
 import cases as C
 from tests_support import make_cfg
 
-REF_UTILS = "/root/reference/data/datasets/utils.py"
-
-
-def _ref():
-    if not os.path.isfile(REF_UTILS):
-        return None
-    spec = importlib.util.spec_from_file_location("_ref_dataset_utils", REF_UTILS)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    return m
-
 
 def test_get_iteration_path(tmp_path):
     from stnerf_b200 import checkpoint_io as io
-    ref = _ref()
+    ref = C.load_golden("checkpoint_io")
     d = str(tmp_path)
     assert io.get_iteration_path(os.path.join(d, "nope")) is None
     assert io.get_iteration_path(d) is None                                   # empty directory
-    for name in ("layered_rfnr_checkpoint_3.pt", "layered_rfnr_checkpoint_12.pt", "layered_rfnr_checkpoint_5_200.pt",
-                 "other.pt"):
+    for name in C.CHECKPOINT_FILE_NAMES:
         open(os.path.join(d, name), "w").close()
     assert io.get_iteration_path(d) == os.path.join(d, "layered_rfnr_checkpoint_12.pt")
     assert io.get_iteration_path(d, fix_iter=7) == os.path.join(d, "frame", "layered_rfnr_checkpoint_7.pt")
-    if ref is not None:
-        assert io.get_iteration_path(d) == ref.get_iteration_path(d)
-        assert io.get_iteration_path(d, 7) == ref.get_iteration_path(d, 7)
-        assert ref.get_iteration_path(os.path.join(d, "nope")) is None
+    assert io.get_iteration_path(d) == os.path.join(d, str(ref["iteration_path"]))
+    assert io.get_iteration_path(d, 7) == os.path.join(d, str(ref["iteration_path_fix7"]))
 
 
 def test_camera_file_parsing(tmp_path):
     from stnerf_b200 import checkpoint_io as io
-    ref = _ref()
-    rs = np.random.RandomState(3)
-    Ks = rs.rand(5, 9) * 1000
+    ref = C.load_golden("checkpoint_io")
+    Ks, poses = C.camera_file_inputs()
     fn = os.path.join(str(tmp_path), "K.txt")
     np.savetxt(fn, Ks)
     got = io.read_intrinsics(fn)
     assert got.shape == (5, 3, 3) and np.array_equal(got, np.loadtxt(fn).reshape(5, 3, 3))
-    poses = rs.rand(5, 12)
     ext = io.campose_to_extrinsic(poses)
     assert ext.shape == (5, 4, 4) and np.array_equal(ext[:, :3, :].reshape(5, 12), poses) and np.all(ext[:, 3] == [0, 0, 0, 1])
     with pytest.raises(Exception):
-        io.campose_to_extrinsic(rs.rand(5, 11))
-    if ref is not None:
-        assert np.array_equal(got, ref.read_intrinsics(fn))
-        assert np.array_equal(ext, ref.campose_to_extrinsic(poses))
+        io.campose_to_extrinsic(np.random.RandomState(3).rand(5, 11))
+    assert np.array_equal(got, ref["intrinsics"])
+    assert np.array_equal(ext, ref["extrinsics"])
 
 
 def test_load_checkpoint_backfills_missing_keys(tmp_path):
